@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- IAF-transform throughput on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload c2a|c2b|...]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload c2a|c2b|...] [--dump-outputs DIR]
 
 A "step" is one fused IAF step (masked-AR conv stack -> mu, s -> z' = (z - .1 mu)/exp(.1 s),
 per-element arw_logsd, per-sample logdet) over one GLOBAL batch of 256 synthetic samples of
@@ -490,7 +490,22 @@ class DeviceBench(object):
         (ms,) = self._max_over_ranks([e0.elapsed_time(e1)])
         direct = self.op.launch_count() - l0
         n_launched = direct if direct else K * self.launches_per_step  # graph replays do not pass through the C ABI
+        self.elbo_scalars = scal
         return ms * 1e-3 / K, int(n_launched), float(scal.sum()), len(groups)
+
+    def last_step_outputs(self, K):
+        """What a caller of the timed path holds after its last step (step K-1): z', arw_logsd and the per-sample logdet of
+        that step, and the ELBO scalar of the evaluation the step closed.  At N > 1 the shards are gathered over ranks
+        (a collective: every rank calls this)."""
+        s = self.sets[(K - 1) % self.nsets]
+        out = {"z_out": s["z_out"], "logsd": s["logsd"], "logdet": s["logdet"]}
+        if self.dist is not None:
+            for k, v in out.items():
+                full = torch.empty((self.world * v.shape[0],) + tuple(v.shape[1:]), device=self.device, dtype=v.dtype)
+                self.dist.all_gather_into_tensor(full, v.contiguous())
+                out[k] = full
+        out["elbo_logdet_sum"] = self.elbo_scalars[-1:]
+        return {k: v.cpu().numpy() for k, v in out.items()}
 
     def training_pair(self, iters=20):
         """Forward that keeps the activations (iaf_step_fwd_train) and backward from them (iaf_step_bwd_saved: gradients of z,
@@ -571,6 +586,24 @@ class DeviceBench(object):
         return t / Ke, Ke, h2d, d2h, check
 
 
+DUMP_LIMIT_BYTES = 64 * 2 ** 20
+
+
+def dump_outputs(d, outs):
+    """Writes ``outs`` as d/<name>.npy.  Arrays with a leading batch axis that together exceed DUMP_LIMIT_BYTES keep a fixed,
+    seeded sample of their rows (the same rows for the same batch size), in ascending order."""
+    batched = [k for k in outs if k != "elbo_logdet_sum"]
+    nb = outs[batched[0]].shape[0]
+    per_row = sum(outs[k].nbytes for k in batched) // nb
+    keep = min(nb, DUMP_LIMIT_BYTES // per_row)
+    if keep < nb:
+        rows = np.sort(np.random.RandomState(0).choice(nb, keep, replace=False))
+        outs = dict(outs, **{k: outs[k][rows] for k in batched})
+    os.makedirs(d, exist_ok=True)
+    for k, v in outs.items():
+        np.save(os.path.join(d, k + ".npy"), np.ascontiguousarray(v, dtype=np.float32))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -583,7 +616,13 @@ def main():
     ap.add_argument("--no-also", action="store_true", help="skip the second headline shape")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--batch", type=int, default=0, help="development: override the workload's global batch")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's outputs as DIR/<name>.npy (float32, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes what the b200 arm computed")
     args.warmup = max(args.warmup, 3)
 
     rank = int(os.environ.get("RANK", "0"))
@@ -625,6 +664,7 @@ def main():
         sampler.phase = "timed"
     t_kernel = db.time_kernels(K)
     t_step, n_launched, elbo_sum, n_groups = db.time_elbo_groups(K)
+    outs = db.last_step_outputs(K) if args.dump_outputs else None
     if sampler:
         sampler.phase = "between"
     elems_step = db.Bg * db.n_z * db.H * db.W
@@ -697,6 +737,8 @@ def main():
         "also": also,
         "elbo_scalar": elbo_sum,
     }
+    if outs is not None:
+        dump_outputs(args.dump_outputs, outs)
     print(json.dumps(line), flush=True)
     if dist is not None:
         dist.destroy_process_group()

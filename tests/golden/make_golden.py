@@ -483,8 +483,10 @@ def main():
             m=rec["m"], s=rec["s"], output=np.asarray(output), kl_obj=np.asarray(kl_obj),
             kl_cost=np.asarray(kl_cost), kl_min=np.float64(kl_min)).items()})
     np.savez_compressed(os.path.join(out_dir, "iaflayer_down.npz"), **down)
+    # the tensor-core shape keeps only what its test reads (inp, context and output would take the file past 1 MB)
     np.savez_compressed(os.path.join(out_dir, "iaflayer_down_tc.npz"), **{k: (v.astype(np.float32) if getattr(v, "ndim", 0) else v)
-                                                                         for k, v in down_tc.items()})
+                                                                         for k, v in down_tc.items()
+                                                                         if k.split("_", 2)[2] not in ("inp", "context", "output")})
 
     # ---- distributions.py (logsumexp / compute_lowerbound / repeat / logps) -----------
     rng = np.random.RandomState(3)
