@@ -46,6 +46,8 @@ SYMBOLS = {
                                           C.POINTER(_P), C.POINTER(_P), C.POINTER(_P), C.c_int, _P]),
     "iaf_multiconv_bwd": (C.c_int, [_P, _P, _P, C.POINTER(_P), C.POINTER(_P), C.POINTER(_P), _P, _P, C.POINTER(_P),
                                     C.POINTER(_P), C.POINTER(_P), C.c_int, _P]),
+    "iaf_multiconv_init": (C.c_int, [_P, _P, _P, C.POINTER(_P), C.POINTER(_P), C.POINTER(_P), C.POINTER(_P), C.POINTER(_P),
+                                     C.POINTER(_P), _P, C.c_int, _P]),
     "iaf_strerror": (C.c_char_p, [C.c_int]),
     "iaf_last_cuda_error": (C.c_char_p, []),
     "iaf_version": (C.c_int, []),

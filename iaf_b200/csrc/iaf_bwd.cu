@@ -17,6 +17,8 @@
 // the Theano variant is the same computation on the point-reflected image (pixel p <-> HW-1-p on every global
 // load/store), its pad channel a position-dependent bias whose gradient is a masked sum of G.
 // Reductions use fixed-order partial sums (no float atomics): results are run-to-run deterministic.
+// The data-dependent initialisation (iaf_multiconv_init, iaf_init_run at the end) also lives here: it runs the stack
+// layer at a time on the same forward layer conv, then per-channel statistics, new parameters and normalised outputs.
 #include "iaf_bwd.h"
 #include "iaf_tc.h"
 
@@ -769,6 +771,154 @@ __global__ void __launch_bounds__(128) iaf_bwd_wnorm_kernel(const __grid_constan
 }
 
 // ------------------------------------------------------------------------------------------
+// data-dependent initialisation (TF layers.py:38-51 with init_scale = 1, Theano ar.py:331-353): per-channel mean and
+// population variance of one stage's pre-activation, the layer's new parameters, and its normalised output.  Values
+// are fp32, accumulation is in double, reductions are fixed-order shared-memory trees (no shuffles, no float
+// atomics): reruns are bit-identical.
+// ------------------------------------------------------------------------------------------
+#define IN_THREADS 256
+
+// sum over the CTA in a fixed order; every thread gets the result
+__device__ __forceinline__ double in_block_sum(double v, double* red) {
+  const int tid = threadIdx.x;
+  red[tid] = v;
+  __syncthreads();
+  for (int s = IN_THREADS / 2; s > 0; s >>= 1) {
+    if (tid < s) red[tid] += red[tid + s];
+    __syncthreads();
+  }
+  const double r = red[0];
+  __syncthreads();  // red is reused by the next call
+  return r;
+}
+
+struct IafInitStatsParams {
+  const float* x;  // [B][planes][HW]
+  double* part;    // [channel][nseg][3]: count, mean, sum of squared deviations of each segment
+  int planes, HW, nseg;
+  long long N;     // B * HW values per channel
+};
+
+// grid (nseg, channels): segment s of a channel's N values (sample-major), two passes over it (mean, then squared
+// deviations from that mean) so a constant channel gives exactly zero
+__global__ void __launch_bounds__(IN_THREADS) iaf_init_stats_kernel(const __grid_constant__ IafInitStatsParams p) {
+  __shared__ double red[IN_THREADS];
+  const int c = blockIdx.y, s = blockIdx.x, tid = threadIdx.x;
+  const long long e0 = p.N * s / p.nseg, e1 = p.N * (s + 1) / p.nseg;
+  const float* xc = p.x + (size_t)c * p.HW;
+  const size_t bstride = (size_t)p.planes * p.HW;
+  double acc = 0.0;
+  for (long long e = e0 + tid; e < e1; e += IN_THREADS) {
+    const long long b = e / p.HW;
+    acc += (double)__ldg(xc + b * bstride + (e - b * p.HW));
+  }
+  const double n = (double)(e1 - e0);
+  const double mean = n > 0.0 ? in_block_sum(acc, red) / n : 0.0;
+  acc = 0.0;
+  for (long long e = e0 + tid; e < e1; e += IN_THREADS) {
+    const long long b = e / p.HW;
+    const double d = (double)__ldg(xc + b * bstride + (e - b * p.HW)) - mean;
+    acc += d * d;
+  }
+  const double m2 = in_block_sum(acc, red);
+  if (tid == 0) {
+    double* q = p.part + ((size_t)c * p.nseg + s) * 3;
+    q[0] = n; q[1] = mean; q[2] = m2;
+  }
+}
+
+struct IafInitLayer {
+  const float* scale_in;  // Theano: kept by a skipped layer
+  const float* bias_in;
+  float* scale_out;
+  float* bias_out;
+  int cout, col0, pairs;  // column of channel co in the stage's output: pairs ? (co/4)*8 + col0 + co%4 : co (iaf_pack.cu)
+};
+
+struct IafInitFinalParams {
+  IafInitLayer layer[IAF_MAX_HEADS];  // one CTA per layer of the stage: the heads stage has one per head
+  const double* part;
+  double* coef;                       // [column][2]: the apply kernel's map out = (x - coef[0]) * coef[1]
+  int* skipped;                       // entry of the stage's first layer, or nullptr
+  int nseg, variant;
+};
+
+__device__ __forceinline__ int in_col(const IafInitLayer& L, int co) { return L.pairs ? (co >> 2) * 8 + L.col0 + (co & 3) : co; }
+
+__global__ void __launch_bounds__(IN_THREADS) iaf_init_finalize_kernel(const __grid_constant__ IafInitFinalParams p) {
+  __shared__ double red[IN_THREADS];
+  const IafInitLayer& L = p.layer[blockIdx.x];
+  const int tid = threadIdx.x;
+  const bool tf = p.variant == IAF_VARIANT_TF;
+  double nzero = 0.0;
+  for (int co = tid; co < L.cout; co += IN_THREADS) {
+    const int col = in_col(L, co);
+    // the segments' (count, mean, M2) merged in order (Chan, Golub & LeVeque's pairwise update)
+    double n = 0.0, mean = 0.0, m2 = 0.0;
+    for (int s = 0; s < p.nseg; ++s) {
+      const double* q = p.part + ((size_t)col * p.nseg + s) * 3;
+      if (q[0] == 0.0) continue;
+      const double nn = n + q[0], dl = q[1] - mean;
+      mean += dl * (q[0] / nn);
+      m2 += q[2] + dl * dl * (n * q[0] / nn);
+      n = nn;
+    }
+    const double var = m2 / n;  // population variance: tf.nn.moments, Theano std (ddof 0)
+    if (!tf && var == 0.0) nzero += 1.0;
+    p.coef[2 * col] = mean;
+    p.coef[2 * col + 1] = 1.0 / sqrt(tf ? var + 1e-10 : var);  // layers.py:46 | ar.py:333 (inf when std = 0: skipped below)
+  }
+  // Theano: a layer with any zero-std channel keeps its parameters and returns h unchanged (ar.py:334-336)
+  const double nzero_all = in_block_sum(nzero, red);
+  const bool skip = nzero_all > 0.0;
+  for (int co = tid; co < L.cout; co += IN_THREADS) {
+    const int col = in_col(L, co);
+    double* k = p.coef + 2 * col;
+    if (skip) {
+      L.scale_out[co] = L.scale_in[co];
+      L.bias_out[co] = L.bias_in[co];
+      k[0] = 0.0;
+      k[1] = 1.0;
+    } else {
+      // TF: g = log(scale) / 3, b = -m * scale (layers.py:47-48); Theano: s = -log(std) / 3, b = -mean(h / std)
+      // (ar.py:339,348-350)
+      L.scale_out[co] = (float)(log(k[1]) / 3.0);
+      L.bias_out[co] = (float)(-k[0] * k[1]);
+    }
+  }
+  if (tid == 0 && p.skipped) p.skipped[blockIdx.x] = (int)nzero_all;
+}
+
+struct IafInitApplyParams {
+  const float* pre;     // [B][planes][HW]: the stage's pre-activation
+  const double* coef;
+  const float* ctx;     // first hidden layer: [B][cout][HW], else nullptr
+  float* out[IAF_MAX_HEADS];  // hidden stage: out[0] = the next stage's input; heads: one per head (nullptr: not wanted)
+  int n_out, cout, pairs, planes, B, HW;
+  int nl;               // hidden stage: the nonlinearity; heads: IAF_NL_NONE
+};
+
+// out = nl((pre - mean) / std (+ context)) on hidden layers (layers.py:161-166, ar.py:400-409); heads: no context, no nl
+__global__ void __launch_bounds__(IN_THREADS) iaf_init_apply_kernel(const __grid_constant__ IafInitApplyParams p) {
+  const size_t per = (size_t)p.B * p.cout * p.HW;
+  const size_t total = per * p.n_out;
+  for (size_t i = (size_t)blockIdx.x * IN_THREADS + threadIdx.x; i < total; i += (size_t)gridDim.x * IN_THREADS) {
+    const int k = (int)(i / per);
+    const size_t r = i - k * per;
+    float* out = p.out[k];
+    if (!out) continue;
+    const int b = (int)(r / ((size_t)p.cout * p.HW));
+    const size_t r2 = r - (size_t)b * p.cout * p.HW;
+    const int co = (int)(r2 / p.HW), px = (int)(r2 - (size_t)co * p.HW);
+    const int col = p.pairs ? (co >> 2) * 8 + 4 * k + (co & 3) : co;
+    const float x = __ldg(p.pre + ((size_t)b * p.planes + col) * p.HW + px);
+    float v = (float)(((double)x - p.coef[2 * col]) * p.coef[2 * col + 1]);
+    if (p.ctx) v += __ldg(p.ctx + r);
+    out[r] = bw_apply_nl(v, p.nl);
+  }
+}
+
+// ------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------
 static int bw_round_up(int a, int b) { return (a + b - 1) / b * b; }
@@ -797,6 +947,9 @@ struct IafBwdPlan {
   IafDgPlan* dg;               // data gradient on the tensor cores (nullptr: exact-fp32 SIMT lconv kernels)
   int wg_tc;                   // weight gradient on the tensor cores too (IAF_BWD_WG_TC=0: the SIMT kernel)
   float* bpart;                // [BW_BIAS_SEG][5][max ncol]: bias / pad-channel partial sums of that path
+  double* ini_part;            // data-dependent init: per-segment statistics [max ncol][nseg][3] (allocated on first use)
+  size_t ini_part_n;
+  double* ini_coef;            // [max ncol][2]
 };
 
 static void bw_free_scratch(IafBwdPlan* pl) {
@@ -885,6 +1038,8 @@ void iaf_bwd_plan_destroy(IafBwdPlan* pl) {
   if (!pl) return;
   if (pl->dg) iaf_dg_plan_destroy(pl->dg);
   if (pl->bpart) cudaFree(pl->bpart);
+  if (pl->ini_part) cudaFree(pl->ini_part);
+  if (pl->ini_coef) cudaFree(pl->ini_coef);
   bw_free_scratch(pl);
   for (int j = 0; j < IAF_MAX_STAGES; ++j)
     if (pl->dwp[j]) cudaFree(pl->dwp[j]);
@@ -1171,6 +1326,103 @@ int iaf_bwd_run(IafBwdPlan* pl, const IafBwdArgs* a, cudaStream_t stream, int* n
     IAF_LAUNCH(iaf_bwd_wnorm_kernel, dim3(max_cout, q.n_layers), 128, 0, stream, q);
     if (cudaGetLastError() != cudaSuccess) return IAF_ERR_CUDA;
     ++nl_;
+  }
+  if (n_launches) *n_launches = nl_;
+  return IAF_OK;
+}
+
+// Data-dependent initialisation, one stage at a time: conv (pre-activation epilogue), statistics, parameters, output.
+// It runs on these exact-fp32 kernels for every plan, tensor-core plans included: it runs once per training run, on one
+// batch, and its statistics become the model's parameters.
+int iaf_init_run(IafBwdPlan* pl, const IafInitArgs* a, cudaStream_t stream, int* n_launches) {
+  const iaf_desc_t& d = pl->d;
+  const int B = a->B, HW = d.H * d.W;
+  const int nst = pl->n_stages, last = nst - 1;
+  const int flip = d.variant == IAF_VARIANT_THEANO ? 1 : 0;
+  int st = bw_ensure_scratch(pl, B);
+  if (st != IAF_OK) return st;
+  // statistics segments of about 4096 values, at most 64 per channel (a function of the shape only: the merge order,
+  // and so every bit of the result, is the same on every run)
+  const long long N = (long long)B * HW;
+  const int nseg = (int)std::min<long long>(64, std::max<long long>(1, N / 4096));
+  int maxcol = 0;
+  for (int j = 0; j < nst; ++j) maxcol = std::max(maxcol, pl->ncol[j]);
+  const size_t npart = (size_t)maxcol * nseg * 3;
+  if (npart > pl->ini_part_n) {
+    if (pl->ini_part) cudaFree(pl->ini_part);
+    pl->ini_part = nullptr;
+    pl->ini_part_n = 0;
+    if (cudaMalloc(&pl->ini_part, sizeof(double) * npart) != cudaSuccess) return IAF_ERR_CUDA;
+    pl->ini_part_n = npart;
+  }
+  if (!pl->ini_coef && cudaMalloc(&pl->ini_coef, sizeof(double) * 2 * maxcol) != cudaSuccess) {
+    pl->ini_coef = nullptr;
+    return IAF_ERR_CUDA;
+  }
+  int nl_ = 0;
+  const float* xin = a->z;
+  for (int j = 0; j < nst; ++j) {
+    const bool heads = j == last;
+    const int planes = heads ? pl->ncol[j] : pl->cout[j];  // heads keep the packed (interleaved) column order
+    float* pre = heads ? pl->hb : pl->G[0];
+    {  // the heads' epilogue writes the pre-activation: bias and pad channel, no context, no nl
+      IafLconvParams q;
+      memset(&q, 0, sizeof(q));
+      q.in = xin;
+      q.w = a->w_packed[j]; q.bias = a->bias_packed[j];
+      q.padw = flip ? a->padw_packed[j] : nullptr;
+      q.out = pre;
+      q.B = B; q.H = d.H; q.W = d.W; q.cin = pl->cin[j]; q.in_planes = pl->cin[j];
+      q.ncol = pl->ncol[j]; q.nout = planes; q.out_planes = planes;
+      q.bwd = 0; q.epi = EPI_FWD_HEADS; q.nl = d.nl; q.flip = flip;
+      if ((st = bw_lconv(pl, q, stream)) != IAF_OK) return st;
+    }
+    IafInitStatsParams sp;
+    memset(&sp, 0, sizeof(sp));
+    sp.x = pre; sp.part = pl->ini_part; sp.planes = planes; sp.HW = HW; sp.nseg = nseg; sp.N = N;
+    IAF_LAUNCH(iaf_init_stats_kernel, dim3(nseg, planes), IN_THREADS, 0, stream, sp);
+    if (cudaGetLastError() != cudaSuccess) return IAF_ERR_CUDA;
+
+    const int nlay = heads ? d.n_heads : 1;
+    const int i0 = heads ? d.n_hidden : j;  // index of the stage's first layer in the parameter arrays
+    IafInitFinalParams fp;
+    memset(&fp, 0, sizeof(fp));
+    for (int k = 0; k < nlay; ++k) {
+      IafInitLayer& L = fp.layer[k];
+      L.scale_in = flip ? a->scale_in[i0 + k] : nullptr;
+      L.bias_in = flip ? a->bias_in[i0 + k] : nullptr;
+      L.scale_out = a->scale_out[i0 + k];
+      L.bias_out = a->bias_out[i0 + k];
+      L.cout = heads ? d.head[k] : d.hidden[j];
+      L.pairs = heads && d.n_heads == 2;
+      L.col0 = 4 * k;
+    }
+    fp.part = pl->ini_part; fp.coef = pl->ini_coef;
+    fp.skipped = a->skipped ? a->skipped + i0 : nullptr;
+    fp.nseg = nseg; fp.variant = d.variant;
+    IAF_LAUNCH(iaf_init_finalize_kernel, nlay, IN_THREADS, 0, stream, fp);
+    if (cudaGetLastError() != cudaSuccess) return IAF_ERR_CUDA;
+    nl_ += 3;
+
+    if (heads && !a->outs) break;
+    IafInitApplyParams ap;
+    memset(&ap, 0, sizeof(ap));
+    ap.pre = pre; ap.coef = pl->ini_coef;
+    ap.planes = planes; ap.B = B; ap.HW = HW;
+    if (heads) {
+      for (int k = 0; k < d.n_heads; ++k) ap.out[k] = a->outs[k];
+      ap.n_out = d.n_heads; ap.cout = d.head[0]; ap.pairs = d.n_heads == 2; ap.nl = IAF_NL_NONE;
+    } else {
+      ap.ctx = j == 0 ? a->ctx : nullptr;
+      ap.out[0] = pl->h[j + 1];
+      ap.n_out = 1; ap.cout = d.hidden[j]; ap.nl = d.nl;
+    }
+    const size_t total = (size_t)ap.n_out * B * ap.cout * HW;
+    IAF_LAUNCH(iaf_init_apply_kernel, (int)std::min<size_t>(592, (total + IN_THREADS - 1) / IN_THREADS), IN_THREADS, 0,
+               stream, ap);
+    if (cudaGetLastError() != cudaSuccess) return IAF_ERR_CUDA;
+    ++nl_;
+    xin = pl->h[j + 1];
   }
   if (n_launches) *n_launches = nl_;
   return IAF_OK;

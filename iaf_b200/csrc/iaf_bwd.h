@@ -45,6 +45,25 @@ struct IafBwdArgs {
   float* const* g_bias;
 };
 
+// Data-dependent initialisation (iaf_multiconv_init): the stack run once, stage by stage, on the exact-fp32 layer conv;
+// each layer's per-channel statistics become its new (g|s, b) and its normalised output feeds the next layer.
+struct IafInitArgs {
+  int B;
+  const float* z;
+  const float* ctx;
+  // every stage packed with TF: zero gain and bias | Theano: the current s and b (iaf_pack.cu layout)
+  const float* w_packed[IAF_MAX_STAGES];
+  const float* bias_packed[IAF_MAX_STAGES];
+  const float* padw_packed[IAF_MAX_STAGES];
+  const float* const* scale_in;  // Theano: copied to the outputs of a skipped layer; unused for TF
+  const float* const* bias_in;
+  float* const* scale_out;       // one entry per layer (hidden layers first, then heads)
+  float* const* bias_out;
+  float* const* outs;            // head outputs of the pass, nullable
+  int* skipped;                  // [n_layers]: channels with zero std (Theano skips the layer when > 0), nullable
+};
+int iaf_init_run(IafBwdPlan* p, const IafInitArgs* a, cudaStream_t stream, int* n_launches);
+
 // allow_tc: the plan's forward runs on the tensor-core path, so its backward may too (data gradient as a layered-kernel stage,
 // weight gradient as MN-major MMAs over the slot stream); a plan pinned to the exact-fp32 SIMT path keeps the SIMT backward
 int iaf_bwd_plan_create(IafBwdPlan** out, const iaf_desc_t* d, const int* cin, const int* cout, const int* cout_pad,

@@ -83,6 +83,8 @@ struct iaf_plan {
   // recompute of iaf_step_bwd (the entry without kept activations) on the forward's own tensor-core kernels
   float* rc_zo; float* rc_ls; float* rc_h[IAF_MAX_HIDDEN];
   int rc_B;
+  // zero gain and bias the TF data-dependent init packs with (allocated on first use)
+  float* init_zeros;
   uint64_t launches;
   // a plan's scratch (partial sums, counters, packed weights, operand images) serves ONE stream at a time: when a call
   // arrives on a different stream than the previous one, the new stream first waits for the old one's work
@@ -305,18 +307,15 @@ void iaf_plan_destroy(iaf_plan_t* pl) {
   if (pl->rc_ls) cudaFree(pl->rc_ls);
   for (int j = 0; j < IAF_MAX_HIDDEN; ++j)
     if (pl->rc_h[j]) cudaFree(pl->rc_h[j]);
+  if (pl->init_zeros) cudaFree(pl->init_zeros);
   delete pl;
 }
 
-int iaf_pack_weights(iaf_plan_t* pl, const float* const* w, const float* const* scale, const float* const* bias,
-                     void* stream_) {
-  if (!pl || !w || !scale || !bias) return IAF_ERR_BAD_ARG;
-  cudaStream_t stream = (cudaStream_t)stream_;
+// the SIMT packed layout of every stage (iaf_pack.cu), from raw parameters
+static int pack_simt(iaf_plan* pl, const float* const* w, const float* const* scale, const float* const* bias,
+                     cudaStream_t stream) {
   const iaf_desc_t& d = pl->d;
   const int n_layers = d.n_hidden + d.n_heads;
-  for (int i = 0; i < n_layers; ++i)
-    if (!w[i] || !scale[i] || !bias[i]) return IAF_ERR_BAD_ARG;
-  { int hs = stream_handoff(pl, stream); if (hs != IAF_OK) return hs; }
   IafPackParams pp;
   memset(&pp, 0, sizeof(pp));
   pp.n_layers = n_layers;
@@ -345,6 +344,19 @@ int iaf_pack_weights(iaf_plan_t* pl, const float* const* w, const float* const* 
   }
   CK(iaf_launch_pack(pp, max_cout, stream));
   pl->launches += 1;
+  return IAF_OK;
+}
+
+int iaf_pack_weights(iaf_plan_t* pl, const float* const* w, const float* const* scale, const float* const* bias,
+                     void* stream_) {
+  if (!pl || !w || !scale || !bias) return IAF_ERR_BAD_ARG;
+  cudaStream_t stream = (cudaStream_t)stream_;
+  const iaf_desc_t& d = pl->d;
+  const int n_layers = d.n_hidden + d.n_heads;
+  for (int i = 0; i < n_layers; ++i)
+    if (!w[i] || !scale[i] || !bias[i]) return IAF_ERR_BAD_ARG;
+  { int hs = stream_handoff(pl, stream); if (hs != IAF_OK) return hs; }
+  { int st = pack_simt(pl, w, scale, bias, stream); if (st != IAF_OK) return st; }
   if (pl->tc) {
     int st = iaf_tc_pack(pl->tc, w, scale, bias, stream);
     if (st != IAF_OK) return st == IAF_ERR_CUDA ? cuda_fail(cudaGetLastError(), "iaf_tc_pack") : st;
@@ -615,6 +627,60 @@ int iaf_multiconv_bwd(iaf_plan_t* pl, const float* z, const float* context, cons
   if (pl->d.n_heads == 2 && !g_outs[1]) return IAF_ERR_BAD_ARG;
   return run_bwd(pl, IAF_MODE_MULTICONV, z, context, w, scale, nullptr, nullptr, nullptr, g_outs, g_z, g_context, g_w,
                  g_scale, g_bias, B, (cudaStream_t)stream);
+}
+
+int iaf_multiconv_init(iaf_plan_t* pl, const float* z, const float* context, const float* const* w,
+                       const float* const* scale, const float* const* bias, float* const* scale_out,
+                       float* const* bias_out, float* const* outs, int* skipped, int B, void* stream_) {
+  if (!pl || !z || !w || !scale_out || !bias_out) return IAF_ERR_BAD_ARG;
+  const iaf_desc_t& d = pl->d;
+  const bool theano = d.variant == IAF_VARIANT_THEANO;
+  if (d.n_hidden > 0 && !context) return IAF_ERR_BAD_ARG;
+  if (theano && (!scale || !bias)) return IAF_ERR_BAD_ARG;
+  if (B <= 0) return IAF_ERR_BAD_ARG;
+  const int n_layers = d.n_hidden + d.n_heads;
+  for (int i = 0; i < n_layers; ++i) {
+    if (!w[i] || !scale_out[i] || !bias_out[i] || scale_out[i] == bias_out[i]) return IAF_ERR_BAD_ARG;
+    if (theano && (!scale[i] || !bias[i])) return IAF_ERR_BAD_ARG;
+    if (theano && (scale_out[i] == scale[i] || bias_out[i] == bias[i])) return IAF_ERR_BAD_ARG;  // outputs never alias inputs
+  }
+  if (outs)
+    for (int k = 0; k < d.n_heads; ++k)
+      if (!outs[k]) return IAF_ERR_BAD_ARG;
+  cudaStream_t stream = (cudaStream_t)stream_;
+  { int hs = stream_handoff(pl, stream); if (hs != IAF_OK) return hs; }
+  // the packed buffers are this pass's scratch: forward and backward entries refuse the plan until it is packed again
+  pl->packed = false;
+  if (!pl->bwd) {
+    int st = iaf_bwd_plan_create(&pl->bwd, &d, pl->cin, pl->cout, pl->cout_pad, pl->head_pad, pl->path == IAF_PATH_TC);
+    if (st != IAF_OK) return st == IAF_ERR_CUDA ? cuda_fail(cudaGetLastError(), "iaf_bwd_plan_create") : st;
+  }
+  // TF: the init branch convolves with l2_normalize(mask o V) alone (layers.py:44-45), i.e. gain exp(0) and bias 0
+  const float* zs[IAF_MAX_HIDDEN + IAF_MAX_HEADS];
+  if (!theano) {
+    int mc = 0;
+    for (int j = 0; j < pl->n_stages; ++j) mc = std::max(mc, pl->cout[j]);
+    if (!pl->init_zeros && cudaMalloc(&pl->init_zeros, sizeof(float) * mc) != cudaSuccess) {
+      pl->init_zeros = nullptr;
+      return cuda_fail(cudaGetLastError(), "cudaMalloc(init zeros)");
+    }
+    CK(cudaMemsetAsync(pl->init_zeros, 0, sizeof(float) * mc, stream));
+    for (int i = 0; i < n_layers; ++i) zs[i] = pl->init_zeros;
+  }
+  { int st = pack_simt(pl, w, theano ? scale : zs, theano ? bias : zs, stream); if (st != IAF_OK) return st; }
+  IafInitArgs a;
+  memset(&a, 0, sizeof(a));
+  a.B = B; a.z = z; a.ctx = context;
+  for (int j = 0; j < pl->n_stages; ++j) {
+    a.w_packed[j] = pl->w[j]; a.bias_packed[j] = pl->bias[j]; a.padw_packed[j] = pl->padw[j];
+  }
+  a.scale_in = scale; a.bias_in = bias; a.scale_out = scale_out; a.bias_out = bias_out;
+  a.outs = outs; a.skipped = skipped;
+  int nl = 0;
+  int st = iaf_init_run(pl->bwd, &a, stream, &nl);
+  if (st == IAF_ERR_CUDA) return cuda_fail(cudaGetLastError(), "iaf_init_run");
+  pl->launches += nl;
+  return st;
 }
 
 int iaf_step_fwd_host(iaf_plan_t* pl, const float* z_host, const float* context_host, float* z_out_host,

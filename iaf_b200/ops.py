@@ -17,6 +17,7 @@ when a parameter tensor changes (SURVEY F9).
 """
 import ctypes as C
 import os
+import warnings
 
 import numpy as np
 import torch
@@ -118,8 +119,9 @@ class IAFOperator(object):
         return any(t.requires_grad for t in ts)
 
     # ---- plans ----------------------------------------------------------------------
-    def _plan(self, H, W, device, layers=None):
-        """Plan for (H, W, device) with the packed weights of ``layers`` (default: the current set_weights())."""
+    def _plan(self, H, W, device, layers=None, pack=True):
+        """Plan for (H, W, device) with the packed weights of ``layers`` (default: the current set_weights());
+        ``pack=False``: the plan as it is (data_init packs for itself)."""
         key = (H, W, device.index)
         ent = self._plans.get(key)
         if ent is None:
@@ -140,6 +142,8 @@ class IAFOperator(object):
                 _lib.check(self._lib.iaf_plan_create(C.byref(handle), C.byref(d)))
             ent = [handle, None]
             self._plans[key] = ent
+        if not pack:
+            return ent[0]
         if layers is None:
             layers = self._layers
         if layers is None:
@@ -235,6 +239,43 @@ class IAFOperator(object):
         out = self._step_raw(z, context, want_logsd, want_logdet or self.checknan == "raise")
         self._nan_guard(out[2])
         return out[0], out[1], (out[2] if want_logdet else None)
+
+    def data_init(self, z, context, names=None):
+        """Data-dependent initialisation on one batch (iaf_multiconv_init): the pass the reference runs once before
+        training -- TF ``init=True`` (layers.py:38-51), Theano ``w['__init']`` (ar.py:331-353).  Writes the new g|s and
+        b into the bound parameter tensors in place (``copy_``), so the next call re-packs; returns the pass's head
+        outputs.  Theano layers with a zero-std channel keep their parameters and warn with the reference's text;
+        ``names`` (one per layer, hidden layers first) are the layer names that text uses."""
+        if self._layers is None:
+            raise RuntimeError("IAFOperator.set_weights() has not been called")
+        n = len(self._layers)
+        if names is None:
+            names = ["layer_%d" % i for i in range(len(self.hidden))] + ["layer_out_%d" % k for k in range(len(self.heads))]
+        with torch.no_grad():
+            z, context, B, H, W = self._shapes(z, context)
+            dev = z.device
+            plan = self._plan(H, W, dev, pack=False)
+            new_s = [torch.empty_like(l[1]) for l in self._layers]
+            new_b = [torch.empty_like(l[2]) for l in self._layers]
+            outs = [torch.empty((B, h, H, W), device=dev, dtype=torch.float32) for h in self.heads]
+            skipped = torch.zeros((n,), device=dev, dtype=torch.int32)
+            arr = lambda ts: (C.c_void_p * n)(*[t.data_ptr() for t in ts])
+            cur = (arr([l[1] for l in self._layers]), arr([l[2] for l in self._layers])) if self.variant == "theano" \
+                else (None, None)  # TF: the init branch does not read g, b
+            self._plans[(H, W, dev.index)][1] = None  # the init pass uses the packed buffers as scratch
+            with torch.cuda.device(dev):
+                _lib.check(self._lib.iaf_multiconv_init(plan, _ptr(z), _ptr(context), arr([l[0] for l in self._layers]),
+                                                        cur[0], cur[1], arr(new_s), arr(new_b),
+                                                        (C.c_void_p * len(outs))(*[o.data_ptr() for o in outs]),
+                                                        _ptr(skipped), B, _stream(dev)))
+            for l, s, b in zip(self._layers, new_s, new_b):
+                l[1].copy_(s)  # bumps _version: every plan of this operator re-packs on its next call
+                l[2].copy_(b)
+            for name, nzero in zip(names, skipped.tolist()):
+                if nzero > 0:  # ar.py:336
+                    warnings.warn("Stdev=0 for %d features in %s. Skipping data-dependent init." % (nzero, name),
+                                  RuntimeWarning)
+        return outs
 
     def _nan_guard(self, logdet):
         if self.checknan == "raise" and bool(torch.isnan(logdet.detach().sum())):
@@ -536,11 +577,20 @@ def _nl_name(nl):
     return nl
 
 
-def ar_multiconv2d(name, x, context, n_h, n_out, nl="elu", params=None, path="auto", **_):
+def ar_multiconv2d(name, x, context, n_h, n_out, nl="elu", params=None, path="auto", init=False, **_):
     """Drop-in for tf_utils/layers.py:ar_multiconv2d -> list of tensors (one per n_out entry).
-    ``params`` stands in for the TF variable scope: a dict holding V/g/b under the TF names."""
+    ``params`` stands in for the TF variable scope: a dict holding V/g/b under the TF names.
+    ``init=True`` is the data-dependent initialisation the reference runs once under ``arg_scope(..., init=True)``
+    (layers.py:38-51): g and b are created in ``params`` where absent, set from this batch's statistics, and the
+    init pass's outputs are returned."""
     if params is None:
         raise ValueError("params (the variable store) is required in eager mode")
+    if init:
+        scopes = [("layer_%d" % i, s) for i, s in enumerate(n_h)] + [("layer_out_%d" % i, s) for i, s in enumerate(n_out)]
+        for scope, size in scopes:
+            for k in "gb":
+                if "%s/%s/%s" % (name, scope, k) not in params and "%s/%s" % (scope, k) not in params:
+                    params["%s/%s/%s" % (name, scope, k)] = torch.zeros(int(size), device=x.device)
     nl = _nl_name(nl)
     # one operator (plans + packed weights) per distinct call site; the parameters are re-bound on every call, so two
     # variable stores sharing a scope name stay correct (they re-pack when they alternate) and nothing is keyed on
@@ -553,6 +603,9 @@ def ar_multiconv2d(name, x, context, n_h, n_out, nl="elu", params=None, path="au
             _TF_OPS.pop(next(iter(_TF_OPS)))  # least recently used
     _TF_OPS[key] = op  # (re-)insert as most recently used
     op.set_weights(_tf_layers(name, params, n_h, n_out))
+    if init:
+        return op.data_init(x, context, names=["%s/layer_%d" % (name, i) for i in range(len(n_h))] +
+                            ["%s/layer_out_%d" % (name, i) for i in range(len(n_out))])
     return op.multiconv(x, context)
 
 
@@ -599,7 +652,10 @@ def multiconv2d(name, n_in, n_h, n_out, size_kernel=(3, 3), flipmask=False, nl="
         if return_hiddens:
             raise NotImplementedError("return_hiddens=True: hidden activations never leave the SM in the fused kernel")
         op.set_weights([(w[n + "_w"], w[n + "_s"], w[n + "_b"]) for n in names])
-        out = op.multiconv(h, context)
+        if "__init" in w:  # ar.py:331-353: data-dependent init, w[..._s] / w[..._b] updated in place (set_value)
+            out = op.data_init(h, context, names=names)
+        else:
+            out = op.multiconv(h, context)
         if len(n_out) == 1:
             out = out[0]  # ar.py:411
         return out

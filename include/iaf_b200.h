@@ -213,6 +213,30 @@ int iaf_multiconv_bwd(iaf_plan_t* plan, const float* z, const float* context, co
                       float* g_context, float* const* g_w, float* const* g_scale,
                       float* const* g_bias, int B, void* stream);
 
+/*
+ * Data-dependent initialisation of the stack: the pass both reference front-ends run once on the first minibatch
+ * before training (tf_train.py:226-228 -> layers.py:38-51 with init_scale = 1; models.py:541-544 -> ar.py:331-353),
+ * layer by layer, each layer's returned tensor feeding the next (context added after hidden layer 0, nl after every
+ * hidden layer).  Statistics are per output channel over (batch, H, W), population variance.
+ *   TF:     x = xcorr(x_in, l2_normalize(mask o V)) (no gain, no bias; the current g, b are not read);
+ *           scale = 1/sqrt(var + 1e-10); g := log(scale)/3; b := -mean*scale; returns scale*(x - mean).
+ *           A zero-variance channel gets scale 1e5.  The forward uses exp(g), not exp(3g) (layers.py:60): a forward with
+ *           the new parameters does NOT reproduce this pass's output -- the reference's behaviour, kept.
+ *   Theano: h = the normal forward of the layer with the CURRENT s and b; if any channel has std 0 the layer keeps s, b
+ *           and returns h (the reference prints a warning); else s := -log(std)/3, h /= std, b := -mean(h), h -= mean(h).
+ *           s and b are overwritten, not composed with their current values.
+ * w/scale/bias: n_hidden + n_heads entries in the layouts of iaf_pack_weights (TF: scale and bias may be NULL, they are
+ * not read).  scale_out/bias_out: the new parameters, same layouts; they must not alias any input.  outs[k]
+ * [B,head[k],H,W]: the pass's head outputs (outs may be NULL).  skipped [n_hidden + n_heads] int32 (may be NULL): the
+ * number of zero-std channels of each layer; Theano skipped the layer when it is > 0, TF always writes 0.
+ * Runs on exact-fp32 kernels with fixed-order double reductions on every plan (tensor-core plans included: it runs once
+ * per training run and its statistics become the parameters); results are bit-identical across runs and paths.
+ * Afterwards the plan is NOT packed: forward and backward entries return IAF_ERR_NOT_PACKED until iaf_pack_weights.
+ */
+int iaf_multiconv_init(iaf_plan_t* plan, const float* z, const float* context, const float* const* w,
+                       const float* const* scale, const float* const* bias, float* const* scale_out,
+                       float* const* bias_out, float* const* outs, int* skipped, int B, void* stream);
+
 /* introspection */
 const char* iaf_strerror(int status);
 const char* iaf_last_cuda_error(void);          /* message of the last failing CUDA call (thread-local) */
